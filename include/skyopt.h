@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define SKYOPT_ABI_VERSION 3
+#define SKYOPT_ABI_VERSION 4
 
 /* error codes */
 #define SKYOPT_OK 0
@@ -205,7 +205,8 @@ typedef struct SkyoptSlot {
                            image_id dict and of a per-region ssh_proxy_command */
   int32_t pad_;
   double hours;         /* estimated_runtime / 3600 (optimizer.py:320-343) */
-  double node_mult;     /* max(num_nodes - reserved, 0) (optimizer.py:353) */
+  double node_mult;     /* num_nodes; the device takes the reserved nodes of
+                           each candidate off it (SkyoptReservation) */
   double time_value;    /* estimated_runtime, the TIME-mode value (:357) */
 } SkyoptSlot;
 
@@ -263,6 +264,20 @@ typedef struct SkyoptDagResult {
   double objective;   /* best_total_objective */
 } SkyoptDagResult;
 
+/*
+ * Consumable reserved capacity of one (cloud, instance type, zone): the sum
+ * over the reservations that the candidate may use
+ * (Resources.get_reservations_available_resources, resources.py:1785-1812;
+ * aws.py:1490-1519, gcp.py:1419-1438). A COST-objective, non-spot candidate
+ * with a zone is valued hourly * hours * max(num_nodes - available, 0)
+ * (optimizer.py:344-354). The table is sorted by (cloud, inst_id, zone_id)
+ * and has no duplicate keys.
+ */
+typedef struct SkyoptReservation {
+  int32_t cloud, inst_id, zone_id;  /* same ids as SkyoptCandidate / SkyoptBlocked */
+  int32_t available;                /* consumable reserved nodes, summed, > 0 */
+} SkyoptReservation;
+
 typedef struct SkyoptProblem {
   const SkyoptQuery *queries;
   int32_t n_queries;
@@ -280,6 +295,8 @@ typedef struct SkyoptProblem {
   int32_t n_blocked;
   const SkyoptDag *dags;
   int32_t n_dags;
+  const SkyoptReservation *reservations; /* may be NULL when n_reservations == 0 */
+  int32_t n_reservations;
 } SkyoptProblem;
 
 typedef struct SkyoptSolution {

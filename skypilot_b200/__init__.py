@@ -9,6 +9,7 @@ from skypilot_b200 import catalog
 from skypilot_b200 import check
 from skypilot_b200 import clouds
 from skypilot_b200 import exceptions
+from skypilot_b200 import reservations
 from skypilot_b200.dag import Dag
 from skypilot_b200.optimizer import DummyResources
 from skypilot_b200.optimizer import Optimizer
@@ -29,5 +30,5 @@ __version__ = '0.1.0'
 __all__ = [
     'AWS', 'Azure', 'Dag', 'DummyResources', 'GCP', 'Lambda', 'Optimizer',
     'OptimizeTarget', 'Resources', 'Task', 'catalog', 'check', 'clouds',
-    'exceptions', 'optimize', 'optimize_batch'
+    'exceptions', 'optimize', 'optimize_batch', 'reservations'
 ]

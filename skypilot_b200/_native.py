@@ -11,7 +11,7 @@ from typing import Optional
 
 import numpy as np
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 ACC_SET_WORDS = 32
 MAX_CLOUDS = 32
 NONE16 = 0xFFFF
@@ -96,13 +96,18 @@ ZONE_DTYPE = np.dtype([
 ], align=True)
 ZONE_ROWS = 128
 
+RESERVATION_DTYPE = np.dtype([
+    ('cloud', '<i4'), ('inst_id', '<i4'), ('zone_id', '<i4'),
+    ('available', '<i4'),
+], align=True)
+
 DAG_RESULT_DTYPE = np.dtype([
     ('status', '<i4'), ('task_fail', '<i4'), ('objective', '<f8'),
 ], align=True)
 
 _EXPECTED_SIZES = {
     'query': 88, 'scan_result': 32, 'slot': 80, 'blocked': 24, 'task': 24,
-    'dag': 24, 'candidate': 32, 'dag_result': 16
+    'dag': 24, 'candidate': 32, 'dag_result': 16, 'reservation': 16
 }
 assert QUERY_DTYPE.itemsize == _EXPECTED_SIZES['query'], QUERY_DTYPE.itemsize
 assert SCAN_RESULT_DTYPE.itemsize == _EXPECTED_SIZES['scan_result']
@@ -112,6 +117,7 @@ assert TASK_DTYPE.itemsize == _EXPECTED_SIZES['task']
 assert DAG_DTYPE.itemsize == _EXPECTED_SIZES['dag']
 assert CANDIDATE_DTYPE.itemsize == _EXPECTED_SIZES['candidate']
 assert DAG_RESULT_DTYPE.itemsize == _EXPECTED_SIZES['dag_result']
+assert RESERVATION_DTYPE.itemsize == _EXPECTED_SIZES['reservation']
 
 _p = ctypes.c_void_p
 
@@ -142,6 +148,7 @@ class Problem(ctypes.Structure):
         ('tariffs', _p), ('n_tariffs', ctypes.c_int32),
         ('blocked', _p), ('n_blocked', ctypes.c_int32),
         ('dags', _p), ('n_dags', ctypes.c_int32),
+        ('reservations', _p), ('n_reservations', ctypes.c_int32),
     ]
 
 

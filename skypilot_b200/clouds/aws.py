@@ -9,7 +9,8 @@ from skypilot_b200.utils import resources_utils
 @registry.CLOUD_REGISTRY.register
 class AWS(cloud.Cloud):
     """AWS: accelerators are part of the instance type; region-level
-    on-demand candidates, zone-level spot candidates (aws.py:347-370)."""
+    on-demand candidates (zone-level with reservations configured), zone-level
+    spot candidates (aws.py:347-371)."""
     _REPR = 'AWS'
     _CATALOG = 'aws'
     _DEFAULT_IMAGE_GB = 45  # DEFAULT_AMI_GB, sky/clouds/aws.py:59
@@ -21,6 +22,14 @@ class AWS(cloud.Cloud):
         # and it does not concern placement.
         del resources, region
         return {}
+
+    @classmethod
+    def optimize_by_zone(cls) -> bool:
+        """One candidate per zone when reservations are configured
+        (aws.py:369-371, aws_utils.use_reservations): reserved capacity is
+        zonal, so on-demand candidates are priced zone by zone."""
+        from skypilot_b200 import reservations  # pylint: disable=import-outside-toplevel
+        return reservations.use_reservations('aws')
 
     def get_egress_cost(self, num_gigabytes: float) -> float:
         """Tiered $/GB out of AWS (aws.py:667-688)."""

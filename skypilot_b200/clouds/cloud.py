@@ -628,10 +628,12 @@ class Cloud:
             # property of (catalog, cloud), looked up once
             rules = self._rules()
             table = self._view().table
-            ctx = (rules, table, bool(table.has_zone_column),
-                   bool(self.optimize_by_zone()), _late('engine'))
+            ctx = (rules, table, bool(table.has_zone_column), _late('engine'))
             ctxs[self.__class__] = ctx
-        rules, table, has_zone_column, by_zone_always, engine = ctx
+        rules, table, has_zone_column, engine = ctx
+        # read per call: AWS splits by zone while the config enables
+        # reservations (the plan templates are keyed on the config generation)
+        by_zone_always = bool(self.optimize_by_zone())
         plan = SlotPlan()
         use_spot = bool(resources.use_spot)
         if use_spot and not rules.supports_spot:

@@ -195,7 +195,7 @@ int ensure(Ctx *x, size_t dbytes, size_t hbytes) {
 // Everything one call needs, laid out twice (host staging / device).
 struct Plan {
   // sizes
-  int nq = 0, nsets = 0, ns = 0, nt = 0, np = 0, ntar = 0, nb = 0, nd = 0;
+  int nq = 0, nsets = 0, ns = 0, nt = 0, np = 0, ntar = 0, nb = 0, nd = 0, nres = 0;
   int n_groups = 0, n_blocks = 0, rpt = 4, tpb = 1, nsq = 0; bool stream = false; bool queue = false; bool want_finalize = true;
   int64_t n_partials = 0, list_entries = 0, fuzzy_entries = 0;
   int64_t cand_cap = 0;   // expand candidate buffers
@@ -210,6 +210,7 @@ struct Plan {
   size_t in_bytes = 0;
   SkyoptQuery *queries; uint32_t *acc_sets; SkyoptSlot *slots; SkyoptTask *tasks;
   int32_t *parents; double *tariffs; SkyoptBlocked *blocked; SkyoptDag *dags;
+  SkyoptReservation *res;
   ScanQuery *squeries; QueryTest *qtests; ScanGroup *groups; const ScanGroup *host_groups = nullptr; int32_t *partial_base, *partial_count;
   int64_t *list_base, *fuzzy_base, *slot_off, *task_off; int32_t *task_dag;
   // device-only scratch
@@ -234,6 +235,7 @@ void carve_inputs(Plan &P, Carver &c) {
   P.tariffs = c.take<double>(P.ntar);
   P.blocked = c.take<SkyoptBlocked>(P.nb);
   P.dags = c.take<SkyoptDag>(P.nd);
+  P.res = c.take<SkyoptReservation>(P.nres);
   P.squeries = c.take<ScanQuery>(P.nsq);
   P.qtests = c.take<QueryTest>(P.nsq);
   P.groups = c.take<ScanGroup>(P.n_groups);
@@ -342,6 +344,23 @@ int validate_problem(const SkyoptCatalog *cat, const SkyoptProblem *pb) {
         return fail(SKYOPT_EINVAL, "dag %d: chain parent must be the previous task", i);
     }
   }
+  if (pb->n_reservations < 0 || (pb->n_reservations > 0 && !pb->reservations))
+    return fail(SKYOPT_EINVAL, "bad reservation table");
+  for (int i = 0; i < pb->n_reservations; ++i) {
+    const SkyoptReservation &r = pb->reservations[i];
+    if (r.cloud < 0 || r.cloud >= C) return fail(SKYOPT_EINVAL, "reservation %d: bad cloud %d", i, r.cloud);
+    if (r.inst_id < cat->cloud_inst_offsets[r.cloud] || r.inst_id >= cat->cloud_inst_offsets[r.cloud + 1])
+      return fail(SKYOPT_EINVAL, "reservation %d: instance id %d is not of cloud %d", i, r.inst_id, r.cloud);
+    if (r.zone_id < 0 || r.zone_id >= cat->cloud_n_zones[r.cloud])
+      return fail(SKYOPT_EINVAL, "reservation %d: bad zone id %d", i, r.zone_id);
+    if (r.available <= 0) return fail(SKYOPT_EINVAL, "reservation %d: available must be > 0", i);
+    if (i > 0) {
+      const SkyoptReservation &q = pb->reservations[i - 1];
+      const bool ordered = q.cloud < r.cloud || (q.cloud == r.cloud && (q.inst_id < r.inst_id ||
+                           (q.inst_id == r.inst_id && q.zone_id < r.zone_id)));
+      if (!ordered) return fail(SKYOPT_EINVAL, "reservation %d: table not sorted by (cloud, inst_id, zone_id) or not unique", i);
+    }
+  }
   return 0;
 }
 
@@ -350,7 +369,7 @@ int build_plan(SkyoptCatalog *cat, const SkyoptProblem *pb, Ctx *x, Plan &P) {
   const int C = cat->dev.n_clouds;
   P.nq = pb->n_queries; P.nsets = pb->n_acc_sets; P.ns = pb->n_slots;
   P.nt = pb->n_tasks; P.np = pb->n_parents; P.ntar = pb->n_tariffs;
-  P.nb = pb->n_blocked; P.nd = pb->n_dags;
+  P.nb = pb->n_blocked; P.nd = pb->n_dags; P.nres = pb->n_reservations;
 
   std::vector<std::vector<int>> by_cloud(C);
   for (int i = 0; i < P.nq; ++i) by_cloud[pb->queries[i].cloud].push_back(i);
@@ -605,6 +624,7 @@ int build_plan(SkyoptCatalog *cat, const SkyoptProblem *pb, Ctx *x, Plan &P) {
   if (P.ntar) memcpy(P.tariffs, pb->tariffs, sizeof(double) * P.ntar);
   if (P.nb) memcpy(P.blocked, pb->blocked, sizeof(SkyoptBlocked) * P.nb);
   if (P.nd) memcpy(P.dags, pb->dags, sizeof(SkyoptDag) * P.nd);
+  if (P.nres) memcpy(P.res, pb->reservations, sizeof(SkyoptReservation) * P.nres);
   memcpy(P.partial_base, pbase.data(), sizeof(int32_t) * P.nq);
   memcpy(P.partial_count, pcount.data(), sizeof(int32_t) * P.nq);
   memcpy(P.list_base, lbase.data(), sizeof(int64_t) * P.nq);
@@ -763,7 +783,7 @@ int enqueue_fast(SkyoptCatalog *cat, Ctx *x, const Plan &P, bool solve, bool wan
   sa.noprune = (noprune_env || cat->noprune) ? 1u : 0u;
   sa.force_any = (want_scan_results || !solve) ? 1u : 0u;
   ExpandOut ex0{P.slot_count, P.slot_inst, P.cand_region, P.cand_zone, P.cand_pa, P.cand_pb};
-  SolveIn in0{P.slots, P.tasks, P.parents, P.tariffs, P.blocked, P.dags, P.slot_off, P.task_off, ex0, 0};
+  SolveIn in0{P.slots, P.tasks, P.parents, P.tariffs, P.blocked, P.dags, P.slot_off, P.task_off, ex0, 0, P.res, P.nres};
   SolveWork w0{P.tc_ref, P.tc_slot, P.tc_cloud, P.tc_hourly, P.tc_value, P.dp, P.back};
   static const bool split_env = [] { const char *e = getenv("SKYOPT_SPLIT"); return e && atoi(e) != 0; }();
   P.ran_fused = false;
@@ -831,7 +851,7 @@ int enqueue_fast(SkyoptCatalog *cat, Ctx *x, const Plan &P, bool solve, bool wan
   if (!solve) return 0;
   if (!P.n_pieces) CU(cudaMemsetAsync(P.err_out, 0, sizeof(int32_t), st));
   ExpandOut ex{P.slot_count, P.slot_inst, P.cand_region, P.cand_zone, P.cand_pa, P.cand_pb};
-  SolveIn in{P.slots, P.tasks, P.parents, P.tariffs, P.blocked, P.dags, P.slot_off, P.task_off, ex, 0};
+  SolveIn in{P.slots, P.tasks, P.parents, P.tariffs, P.blocked, P.dags, P.slot_off, P.task_off, ex, 0, P.res, P.nres};
   SolveWork w{P.tc_ref, P.tc_slot, P.tc_cloud, P.tc_hourly, P.tc_value, P.dp, P.back};
   if (P.nt) {
     PlaceArgs pa{};
@@ -931,7 +951,7 @@ int enqueue_kernels(SkyoptCatalog *cat, Ctx *x, const Plan &P, bool solve,
   }
   CU(cudaEventRecord(x->ev[3], st));
   if (P.nd) {
-    SolveIn in{P.slots, P.tasks, P.parents, P.tariffs, P.blocked, P.dags, P.slot_off, P.task_off, ex, 0};
+    SolveIn in{P.slots, P.tasks, P.parents, P.tariffs, P.blocked, P.dags, P.slot_off, P.task_off, ex, 0, P.res, P.nres};
     SolveWork w{P.tc_ref, P.tc_slot, P.tc_cloud, P.tc_hourly, P.tc_value, P.dp, P.back};
     SolveOut out{P.chosen, P.chosen_index, P.task_n, P.dagres};
     gather_kernel<<<P.nt, kGatherThreads, 0, st>>>(cat->dev, in, w, P.task_dag, P.task_n);
@@ -1010,7 +1030,7 @@ int copy_solution(SkyoptCatalog *cat, Ctx *x, const Plan &P, const SkyoptProblem
       CU(cudaMalloc(&d_tab, sizeof(SkyoptCandidate) * off[P.nt]));
       CU(cudaMemcpyAsync(d_off, off.data(), sizeof(int64_t) * (P.nt + 1), cudaMemcpyHostToDevice, x->stream));
       ExpandOut ex{P.slot_count, P.slot_inst, P.cand_region, P.cand_zone, P.cand_pa, P.cand_pb};
-      SolveIn in{P.slots, P.tasks, P.parents, P.tariffs, P.blocked, P.dags, P.slot_off, P.task_off, ex, 0};
+      SolveIn in{P.slots, P.tasks, P.parents, P.tariffs, P.blocked, P.dags, P.slot_off, P.task_off, ex, 0, P.res, P.nres};
       SolveWork w{P.tc_ref, P.tc_slot, P.tc_cloud, P.tc_hourly, P.tc_value, P.dp, P.back};
       table_kernel<<<P.nt, 128, 0, x->stream>>>(in, w, P.task_n, P.nt, d_off, d_tab);
       cudaError_t e = cudaGetLastError();
@@ -1537,7 +1557,7 @@ int skyopt_session_resolve(SkyoptSession *s, const SkyoptBlocked *blocked, int n
   CU(cudaEventRecord(x->ev[3], st));
   {
     ExpandOut ex{P.slot_count, P.slot_inst, P.cand_region, P.cand_zone, P.cand_pa, P.cand_pb};
-    SolveIn in{P.slots, P.tasks, P.parents, P.tariffs, P.blocked, P.dags, P.slot_off, P.task_off, ex, 0};
+    SolveIn in{P.slots, P.tasks, P.parents, P.tariffs, P.blocked, P.dags, P.slot_off, P.task_off, ex, 0, P.res, P.nres};
     SolveWork w{P.tc_ref, P.tc_slot, P.tc_cloud, P.tc_hourly, P.tc_value, P.dp, P.back};
     SolveOut out{P.chosen, P.chosen_index, P.task_n, P.dagres};
     gather_kernel<<<P.nt, kGatherThreads, 0, st>>>(cat->dev, in, w, P.task_dag, P.task_n);

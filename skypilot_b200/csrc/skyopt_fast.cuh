@@ -648,7 +648,7 @@ struct PlaceSlot {
   unsigned long long vmin; // price_key of the cheapest unblocked candidate's value
   unsigned long long v2;   // ... of the cheapest one in front of it (kKeyNone: none)
   int32_t vidx;            // first candidate (index in the task) with that value
-  int32_t pad_;
+  int2 res;                // reservation entries [x, y) of (cloud, inst); empty: none
 };
 
 struct PlaceSmem {
@@ -720,6 +720,12 @@ __device__ __forceinline__ void place_body(const PlaceArgs &a, int t, unsigned c
         p.list_n = host.cnt[col];
       }
     }
+    // the slot's reservation entries, searched once: lanes then look up
+    // their candidate's zone inside this range only. Spot candidates and the
+    // TIME objective never consume reserved nodes.
+    p.res = make_int2(0, 0);
+    if (a.in.n_res && TK.minimize_cost && !S.use_spot && p.kind != 0 && p.inst >= 0)
+      p.res = reservation_range(a.in.res, a.in.n_res, S.cloud, p.inst);
     ps[tid] = p;
   }
   __syncthreads();
@@ -823,7 +829,9 @@ __device__ __forceinline__ void place_body(const PlaceArgs &a, int t, unsigned c
           a.w.tc_slot[o] = s;
           a.w.tc_cloud[o] = S.cloud;
           a.w.tc_hourly[o] = hourly;
-          const double value = TK.minimize_cost ? __dmul_rn(__dmul_rn(hourly, S.hours), S.node_mult)
+          double mult = S.node_mult;
+          if (p.res.y > p.res.x && zout >= 0) mult = reserved_node_mult(mult, reserved_in_range(a.in.res, p.res, zout));
+          const double value = TK.minimize_cost ? __dmul_rn(__dmul_rn(hourly, S.hours), mult)
                                                 : S.time_value;
           a.w.tc_value[o] = value;
           const unsigned long long vk = price_key(value);

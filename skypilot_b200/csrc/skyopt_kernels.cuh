@@ -22,6 +22,7 @@
 #include <stdint.h>
 
 #include "skyopt.h"
+#include "skyopt_reserve.cuh"
 
 namespace skyopt {
 
@@ -1346,6 +1347,8 @@ struct SolveIn {
   const int64_t *task_off;   // [n_tasks+1] into the task candidate arrays
   ExpandOut ex;
   int tables_only;           // candidates were given by the caller: no slots
+  const SkyoptReservation *res;  // reserved capacity table (skyopt_reserve.cuh)
+  int32_t n_res;                 // 0 = none: values are hourly * hours * num_nodes
 };
 
 struct SolveWork {
@@ -1433,10 +1436,14 @@ gather_kernel(CatDev cat, SolveIn in, SolveWork w, const int32_t *__restrict__ t
                          (B.use_spot == -1 || B.use_spot == S.use_spot);
           if (m) { keep = false; break; }
         }
-        // float(hourly_cost * hours) * max(num_nodes - reserved, 0)
+        // float(hourly_cost * hours) * max(num_nodes - reserved, 0); spot
+        // and zone-less candidates have no reserved nodes
         hourly = __dadd_rn(in.ex.cand_price_a[ref], in.ex.cand_price_b[ref]);
+        double mult = S.node_mult;
+        if (in.n_res && D.minimize_cost && !S.use_spot && zn >= 0 && inst >= 0)
+          mult = reserved_node_mult(mult, reserved_nodes(in.res, in.n_res, S.cloud, inst, zn));
         value = D.minimize_cost
-                    ? __dmul_rn(__dmul_rn(hourly, S.hours), S.node_mult)
+                    ? __dmul_rn(__dmul_rn(hourly, S.hours), mult)
                     : S.time_value;
         if (keep) {
           // stash the cloud in the low bits of nothing: written below

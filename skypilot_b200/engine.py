@@ -269,6 +269,9 @@ class ProblemBuilder:
         self.tariffs: List[float] = []
         self.blocked: List[Dict[str, int]] = []
         self.dags: List[Dict[str, int]] = []
+        # reserved capacity (reservations.device_table): one table for every
+        # DAG of the batch; None = not stated yet, treated as empty
+        self.reservations: Optional[Tuple[np.ndarray, int]] = None
 
     @property
     def n_queries(self) -> int:
@@ -548,6 +551,10 @@ class PackedProblem:
         self.n_blocked = len(b.blocked)
         self.dags = ProblemBuilder._pack(b.dags, _native.DAG_DTYPE)
         self.n_dags = len(b.dags)
+        if b.reservations is not None and b.reservations[1] > 0:
+            self.reservations, self.n_reservations = b.reservations
+        else:
+            self.reservations, self.n_reservations = None, 0
 
     def c_problem(self) -> _native.Problem:
         p = _native.Problem()
@@ -567,6 +574,9 @@ class PackedProblem:
         p.n_blocked = self.n_blocked
         p.dags = _addr(self.dags)
         p.n_dags = self.n_dags
+        p.reservations = (None if self.reservations is None else
+                          _addr(self.reservations))
+        p.n_reservations = self.n_reservations
         return p
 
     def h2d_bytes(self) -> int:
@@ -575,7 +585,8 @@ class PackedProblem:
                    self.slots.nbytes + self.tasks.nbytes +
                    self.parents.nbytes + self.tariffs.nbytes +
                    self.blocked.nbytes * (self.n_blocked > 0) +
-                   self.dags.nbytes)
+                   self.dags.nbytes +
+                   16 * self.n_reservations)
 
 
 class Solution:

@@ -26,7 +26,9 @@ from skypilot_b200 import clouds
 from skypilot_b200 import dag as dag_lib
 from skypilot_b200 import engine
 from skypilot_b200 import exceptions
+from skypilot_b200 import reservations
 from skypilot_b200 import resources as resources_lib
+from skypilot_b200 import skypilot_config
 from skypilot_b200 import task as task_lib
 from skypilot_b200.utils import resources_utils
 from skypilot_b200.utils import timeline
@@ -490,6 +492,10 @@ class Optimizer:
                 raise_if_no_cloud_access=True)
         store = catalog.get_store()
         b = builder if builder is not None else engine.ProblemBuilder(store)
+        if b.reservations is None:
+            # reserved capacity per (cloud, instance type, zone): one table
+            # for every DAG stated into this builder
+            b.reservations = reservations.device_table(store)
         n_clouds = len(store.clouds)
         cloud_objs = store.__dict__.get('_cloud_objs')
         if cloud_objs is None:
@@ -501,7 +507,10 @@ class Optimizer:
         hints: Dict[Any, Dict[Any, str]] = collections.defaultdict(dict)
         local_index = {t: i for i, t in enumerate(topo_real)}
         task_begin = len(b.tasks)
-        generation = store.__dict__.get('_memo_generation', 0)
+        # a config change re-states tasks (e.g. AWS splits by zone while
+        # reservations are configured)
+        generation = (store.__dict__.get('_memo_generation', 0),
+                      skypilot_config.generation())
         enabled_key = tuple(type(c) for c in enabled)
         for task in topo_real:
             slot_begin = b.n_slots
@@ -1052,6 +1061,8 @@ class OptimizerSession:
         self.quiet = quiet
         self._session: Optional[engine.Session] = None
         self._problem = None
+        # (reservation, config) generations the open session was stated under
+        self._state_key = None
         self._fallback = any(isinstance(t.resources, list) for t in dag.tasks)
 
     def __enter__(self):
@@ -1084,7 +1095,14 @@ class OptimizerSession:
                 raise RuntimeError(
                     'the catalog changed while an OptimizerSession was open; '
                     'close the session and open a new one')
+            state_key = (reservations.generation(),
+                         skypilot_config.generation())
+            if self._session is not None and state_key != self._state_key:
+                # new reservation counts or config: the device-resident
+                # candidate values are stale, state the DAG again
+                self.close()
             if self._session is None:
+                self._state_key = state_key
                 problem = Optimizer._state_problem(  # pylint: disable=protected-access
                     graph, topo_real, self.minimize_cost, blocked,
                     dag.is_chain())

@@ -635,6 +635,20 @@ class Resources:
                 self.accelerators, self.use_spot, self._region, self._zone)
         return float(hourly_cost * hours)
 
+    def get_reservations_available_resources(self) -> Dict[str, int]:
+        """{reservation name: consumable reserved nodes} of this launchable
+        (sky/resources.py:1785-1812); see skypilot_b200/reservations.py."""
+        from skypilot_b200 import reservations  # pylint: disable=import-outside-toplevel
+        if self.use_spot or isinstance(self._cloud, clouds.DummyCloud):
+            return {}
+        assert (self._cloud is not None and self._instance_type is not None
+                and self._region is not None), (
+                    f'Cloud, instance type, region must be specified. '
+                    f'Resources={self}')
+        return reservations.available_resources(
+            str(self._cloud).lower(), self._instance_type, self._region,
+            self._zone, self.use_spot)
+
     def should_be_blocked_by(self, blocked: 'Resources') -> bool:
         """Wildcard match against a blocked entry
         (sky/resources.py:1938-1961): a None field of `blocked` matches

@@ -2,6 +2,21 @@
 # compute-sanitizer over the kernel modes (profiles/round2_sanitizer_*.log).
 mkdir -p gpurun_out/sanitizer
 S=/usr/local/cuda/bin/compute-sanitizer
+if [ "${1:-}" = reservations ]; then
+  # the capacity-reservation suite (tests/golden/reservations.json); logs go
+  # to $SANITIZE_DIR (default: a new temporary directory)
+  D=${SANITIZE_DIR:-$(mktemp -d)}
+  mkdir -p "$D"
+  for mode in auto fast-split; do
+    for tool in memcheck racecheck; do
+      log="$D/${tool}_reservations_${mode}.log"
+      timeout 600 $S --tool $tool --print-limit 20 python tools/sanitize_reservations.py $mode > "$log" 2>&1
+      echo "$tool reservations $mode rc=$? $(grep -E 'ERROR SUMMARY|RACECHECK SUMMARY' "$log" | tail -1)"
+    done
+  done
+  echo "logs in $D"
+  exit 0
+fi
 for mode in auto fast-split fast-noprune tile queue; do
   for tool in memcheck racecheck; do
     timeout 600 $S --tool $tool --print-limit 20 python tools/sanitize_target.py $mode \
